@@ -16,6 +16,7 @@ must equal the single-GPU encode bit for bit.  A mismatch aborts the run: no lin
 oracle/Makefile: AVX2 + OpenMP build, all host threads) on the same config; rank 0 only.
 
 One JSON line on stdout (rank 0).  See DESIGN.md section 7 for how every field is measured.
+`--dump-outputs DIR` also writes a fixed sample of the parity blocks of the last timed step to DIR/parity.npy.
 """
 import argparse
 import ctypes
@@ -34,6 +35,8 @@ METRIC = "rs_encode_GBps_n2^20_k2^19_4KiB_blocks"
 # hash (main.cpp:203-212) of the parity of fill A (data0[i] = i % P), recorded from the unmodified reference: SURVEY.md 8c,
 # tests/golden/survey_8c.json "encode_fillA"; key = (log2 N, words per block)
 GOLDEN_PARITY_HASH_FILL_A = {(7, 1024): 421122310, (11, 1024): 2634925848, (16, 1024): 147925734, (19, 1024): 4272226309, (7, 513): 56723226}
+DUMP_ROWS = 1024                # parity blocks --dump-outputs writes: 8 MiB at 4 KiB blocks
+DUMP_MAX_BYTES = 64 << 20
 
 
 def workload_name(args):
@@ -107,6 +110,8 @@ def parse_args():
                     help="multi-GPU headline: ONE transform sharded over the GPUs with the exchange fused into the kernels' stores (default; strong scaling, "
                          "BASELINE config 4), the same with two NCCL all-to-alls, or only independent stripes (weak scaling)")
     ap.add_argument("--no-stripes", action="store_true", help="skip the secondary independent-stripes measurement of a multi-GPU run")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the parity the last timed step computed to DIR/parity.npy (float64, a fixed "
+                                                          "sample of at most %d blocks; see dump_rows) so two builds can be compared output for output" % DUMP_ROWS)
     return ap.parse_args()
 
 
@@ -240,6 +245,8 @@ def cpu_encode_runner(log_n, size_words, calibrate=True):
 
 
 def run_reference_arm(args):
+    if args.dump_outputs:
+        raise SystemExit("--dump-outputs writes the B200 arm's parity; the reference arm does not support it")
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return 0
@@ -316,6 +323,23 @@ def check_golden(args, h, what):
     if want is not None and h != want:
         raise SystemExit("PARITY FAILURE (%s): hash %d != golden %d of the unmodified reference for N=2^%d, %d-byte blocks" % (what, h, want, key[0], args.block_bytes))
     return {"hash": h, "golden": want, "golden_match": None if want is None else True}
+
+
+def dump_rows(N, S):
+    """Global parity blocks written by --dump-outputs: every block when they fit, otherwise a sorted sample drawn with a fixed
+    seed, so that runs with the same --log-n and --block-bytes write the same blocks."""
+    import numpy as np
+    rows = min(N, DUMP_ROWS, max(1, DUMP_MAX_BYTES // (8 * S)))
+    if rows == N:
+        return np.arange(N)
+    return np.sort(np.random.default_rng(0).choice(N, rows, replace=False))
+
+
+def write_dump(out_dir, sample):
+    """sample: int32 CUDA tensor [rows, S] of parity words -> out_dir/parity.npy as float64 (exact: every word is < P < 2^53)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "parity.npy"), sample.cpu().numpy().view(np.uint32).astype(np.float64))
 
 
 def per_kernel_roofline(fe, data, nbytes, peak, reps):
@@ -414,6 +438,8 @@ def run_single_or_stripes(args, fe, rank, world, local, dev, numa):
         time.sleep(0.25)
     ms, launches = time_stripes(args, fe, dev, world, data)
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:             # data holds the parity of the last timed encode until the roofline loop below
+        write_dump(args.dump_outputs, data[torch.from_numpy(dump_rows(N, S)).to(dev)])
 
     peak, peak_src = measured_peak()
     kernels = per_kernel_roofline(fe, data, nbytes, peak, max(3, min(args.steps, 10))) if rank == 0 else None
@@ -566,6 +592,14 @@ def run_sharded(args, fe, rank, world, local, dev, numa):
     sync()
     if fused:
         enc.check()                             # no barrier timed out: the ranks stayed in step
+    if args.dump_outputs:                       # x: this rank's rows of the last timed encode (global block l*G + rank = row l)
+        g = torch.from_numpy(dump_rows(N, S)).to(dev)
+        owned = g % world == rank
+        sample = torch.zeros((g.numel(), S), dtype=torch.int32, device=dev)
+        sample[owned] = x[g[owned] // world]
+        dist.reduce(sample, dst=0)              # one rank contributes each row, the others zeros
+        if rank == 0:
+            write_dump(args.dump_outputs, sample)
     phases = None
     if fused:                                   # more encodes with events between the phases (max over ranks of the mean per phase)
         names = ["pass_A", "barrier_1", "pass_BC", "barrier_2", "pass_D"]

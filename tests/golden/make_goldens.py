@@ -1,7 +1,8 @@
-"""Regenerates / cross-checks tests/golden/survey_8c.json against the reference compiled in oracle/_ref.
+"""Regenerates / cross-checks tests/golden/survey_8c.json, vectors.npz and reference_outputs.json against the reference
+compiled in oracle/_ref.
 
-Needs /root/reference (this container only).  Usage: python tests/golden/make_goldens.py [--write]
-Without --write it only verifies that the committed file matches what the reference computes here.
+Needs the reference sources when oracle/_ref is built (oracle/Makefile, REF=<path>).  Usage: python tests/golden/make_goldens.py [--write]
+Without --write it only verifies that the committed files match what the reference computes here.
 """
 import json
 import os
@@ -65,6 +66,27 @@ def main():
             if not np.array_equal(old[k], v):
                 bad += 1
                 print("MISMATCH vector", k)
+    # field operations on random pairs, and digests of outputs too large to store, for tests/test_oracle.py
+    rng = np.random.default_rng(3)
+    out = {"gf_pairs": [], "transforms": []}
+    for _ in range(200):
+        x, y = int(rng.integers(0, ol.P)), int(rng.integers(0, ol.P))
+        out["gf_pairs"].append([x, y, r.ref_gf_mul(x, y), r.ref_gf_add(x, y), r.ref_gf_sub(x, y)])
+    for L, S in ((2, 3), (6, 17), (9, 1024), (10, 16), (11, 64), (13, 33)):     # flat / 2-D / cube paths of MFA_NTT
+        a = ol.fill_B(o, 1 << L, S)
+        t = {"L": L, "S": S, "input": ol.sha256(a)}
+        for inv in (0, 1):
+            b = a.copy(); r.ref_mfa_ntt_flat(b.ctypes.data, 1 << L, S, inv); t["ntt%d" % inv] = ol.sha256(b)
+        b = a.copy(); r.ref_rs_encode_flat(b.ctypes.data, 1 << L, S); t["encode"] = ol.sha256(b)
+        out["transforms"].append(t)
+    path = os.path.join(HERE, "reference_outputs.json")
+    if "--write" in sys.argv:
+        with open(path, "w") as f:             # one entry per line
+            f.write("{\n" + ",\n".join('"%s": [\n%s]' % (k, ",\n".join(json.dumps(e) for e in v)) for k, v in out.items()) + "}\n")
+        print("wrote", path)
+    elif json.load(open(path)) != out:
+        bad += 1
+        print("MISMATCH", path)
     print("goldens", "MISMATCH" if bad else "verified against the compiled reference")
     return 1 if bad else 0
 

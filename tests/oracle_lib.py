@@ -1,5 +1,6 @@
 """ctypes loaders for the CPU oracle (oracle/liboracle.so) and the compiled reference (oracle/_ref). Test-only."""
 import ctypes
+import hashlib
 import os
 import subprocess
 
@@ -63,6 +64,11 @@ def fill_A(o, N, S):
 
 def fill_B(o, N, S):
     a = np.empty((N, S), dtype=np.uint32); o.oracle_fill_B(a.ctypes.data, N * S); return a
+
+
+def sha256(a):
+    """Digest of a uint32 array's words (little-endian, row-major): stands for an output buffer too large to store."""
+    return hashlib.sha256(np.ascontiguousarray(a, dtype="<u4").tobytes()).hexdigest()
 
 
 def ohash(o, a):
